@@ -3,10 +3,12 @@
                    modules/video/src/optflowgf.cpp, the function modules/optflow/src/interfaces.cpp:154-157 forwards to)
   tvl1_ref_*.npz   the reference's OWN CPU Dual TV-L1, /root/reference/modules/optflow/src/tvl1flow.cpp compiled
                    unmodified into oracle/_ref/libtvl1_ref.so (oracle/Makefile, oracle/ref_shim/)
+  tvl1_second_input.npz   the same reference build on a second input, once with fixed work (what the C port must
+                   reproduce bit for bit) and once from an initial flow (which the port refuses)
   brox_720p.npz, denselk_1080p.npz   BASELINE-size outputs of the numpy restatements oracle/brox_model.py and
                    oracle/denselk_model.py (no CPU implementation exists upstream: "parity unpinned"), stored as float32
                    on a stride-4 grid plus full-resolution means -- 2 minutes (brox) / 27 minutes (denselk) of numpy
-python tests/golden/make_golden.py [farneback] [tvl1] [brox] [denselk]      (no argument = farneback + tvl1)"""
+python tests/golden/make_golden.py [farneback] [tvl1] [tvl1_second] [brox] [denselk]   (no argument = farneback + tvl1)"""
 import os
 import sys
 
@@ -55,6 +57,22 @@ if "tvl1" in WHAT:
         out.update({"kw_" + k: v for k, v in kw.items()})
         np.savez_compressed(os.path.join(HERE, f"tvl1_ref_{name}.npz"), **out)
         print("tvl1", name, flow.shape, float(np.abs(flow).mean()))
+
+if "tvl1_second" in WHAT:
+    from oracle import tvl1_cpu, tvl1_ref  # noqa: E402
+    fixed = dict(warps=10, epsilon=0.0, innerIterations=1, outerIterations=30, medianFiltering=1)
+    from_init = dict(nscales=1, warps=1, epsilon=0.0, innerIterations=1, outerIterations=2, medianFiltering=1,
+                     useInitialFlow=True)
+    I0, I1, _ = synth.make_pair(150, 190, seed=9, kind="smooth")
+    flow = tvl1_ref.calc(I0, I1, tvl1_cpu.TVL1Params(**fixed))
+    init = np.zeros(I0.shape + (2,), np.float32)
+    init[..., 0] = 1.5
+    flow_init = tvl1_ref.calc(I0, I1, tvl1_cpu.TVL1Params(**from_init), init)
+    out = {"I0": I0, "I1": I1, "flow": flow, "init": init, "flow_init": flow_init}
+    out.update({"kw_" + k: v for k, v in fixed.items()})
+    out.update({"kwinit_" + k: v for k, v in from_init.items()})
+    np.savez_compressed(os.path.join(HERE, "tvl1_second_input.npz"), **out)
+    print("tvl1_second", flow.shape, float(np.abs(flow).mean()), float(flow_init[..., 0].mean()))
 
 
 def _model_fixture(name, I0, I1, flow, kw, seed, kind, dtype):
